@@ -57,7 +57,38 @@ def parse():
                          "GPUs (10248 = level-3 grid x 4 in-plane rotations); 0 = weak scaling, --poses per GPU")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the extra legs (other precision modes, eager-cuDNN baseline, LDM variant)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (similarity rows `sim`, "
+                         "top-5 indices `topi`) as DIR/<name>.npy; the inputs are seeded, so two builds run with the "
+                         "same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the B200 path; the reference arm times a sample of the grid on the host")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy, float32 kept and every other dtype as float64, at most
+    DUMP_LIMIT_BYTES in all: an array that does not fit is replaced by a fixed, seeded sample of its
+    flattened elements (the same sample for the same shape, so runs stay comparable).  The smallest arrays
+    are written first, so only the largest ones are ever sampled."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_LIMIT_BYTES
+    for name, t in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        room = (budget - 4096) // a.itemsize               # 4 KB: the .npy header, generously
+        if a.size > room:
+            keep = np.sort(np.random.default_rng(0).choice(a.size, size=max(room, 0), replace=False))
+            a = a.reshape(-1)[keep]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        budget -= a.nbytes + 4096
 
 
 # ---------------------------------------------------------------------------------------
@@ -467,12 +498,19 @@ def main_ldm(args):
             t = float(tt)
         return t
 
+    last = {}
+
+    def step_kept():                          # the timed step, keeping its result for --dump-outputs
+        last["out"] = step_resident()
+
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(step_resident, args.steps, max(args.warmup, 3))
+    ms = timed(step_kept, args.steps, max(args.warmup, 3))
     launches = m.last_launch_count
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"sim": last["out"]["sim"], "topi": last["out"]["topi"]})
     ms_e2e = timed(step_e2e, args.steps, max(args.warmup, 3))
     m.profile(True)
     step_resident()
@@ -615,6 +653,10 @@ def main():
         return step_resident, step_e2e
 
     step_resident, step_e2e = make_steps(model)
+    last = {}
+
+    def step_kept():                          # the timed step, keeping its result for --dump-outputs
+        last["out"] = step_resident()
 
     def barrier():
         if world > 1:
@@ -643,9 +685,12 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(step_resident, args.steps, max(args.warmup, 3))
+    ms = timed(step_kept, args.steps, max(args.warmup, 3))
     launches_per_step = unet.last_launch_count
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        sim, topi, _ = last["out"]
+        dump_outputs(args.dump_outputs, {"sim": sim, "topi": topi})
     ms_e2e = timed(step_e2e, args.steps, max(args.warmup, 3))
 
     # ---- BASELINE configs[3] beside the weak-scaling headline: the FIXED 10 248-pose grid (level-3 icosphere x 4

@@ -101,6 +101,26 @@ def test_scripts_have_no_undefined_names():
             assert not missing, (script, fn.name, sorted(missing))
 
 
+def test_bench_dump_outputs_keeps_dtypes_and_the_size_cap(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 stays float32, indices become float64, and past the size cap the
+    largest array is replaced by the same seeded sample of its elements on every run."""
+    import numpy as np
+    import bench
+    sim, topi = torch.randn(3, 1000), torch.arange(15).view(3, 5)
+    bench.dump_outputs(str(tmp_path / "full"), {"sim": sim, "topi": topi})
+    a, b = np.load(tmp_path / "full" / "sim.npy"), np.load(tmp_path / "full" / "topi.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, sim.numpy())
+    assert b.dtype == np.float64 and np.array_equal(b, topi.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * 4096 + 2000)
+    for run in ("one", "two"):
+        bench.dump_outputs(str(tmp_path / run), {"sim": sim, "topi": topi})
+    files = [tmp_path / "one" / f for f in ("sim.npy", "topi.npy")]
+    assert sum(f.stat().st_size for f in files) <= bench.DUMP_LIMIT_BYTES
+    s1, s2 = np.load(tmp_path / "one" / "sim.npy"), np.load(tmp_path / "two" / "sim.npy")
+    assert 0 < s1.size < sim.numel() and np.array_equal(s1, s2) and np.isin(s1, sim.numpy()).all()
+    assert np.array_equal(np.load(tmp_path / "one" / "topi.npy"), topi.numpy())
+
+
 def test_both_unets_offer_the_interface_the_sharded_sweep_drives():
     """nope_b200.dist.ShardedSweep calls set_metric() and sweep(query_feat=, want_emb=, want_sim=, k=, idx_base=,
     out=) on whichever UNet it is given; the LDM mirror once lagged behind (multi-GPU LDM sweeps raised)."""

@@ -3,7 +3,7 @@
 #   gpurun --timeout 900 -- 'bash tools/gpu.sh <step> [<step> ...]'
 # steps: fused | unet | tests | ldmtests | time | bench | benchall | launches | ncu_conv | ncu_mem | smoke | sanitize
 # Logs land in gpurun_out/ (merged back by gpurun, < 64 MiB).
-cd "${GRAFT_REPO_ROOT:-/root/repo}"
+cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,clocks.sm,clocks.max.sm,power.draw --format=csv,noheader > gpurun_out/smi.txt 2>&1
 run() { echo "== $1"; shift; timeout "$@"; echo "rc=$?"; }

@@ -4,13 +4,14 @@ Runs the oracle with .half().float() inserted at the points where the CUDA path 
 weights only 9.1e-4, +conv out 1.20e-3, +gn out 1.28e-3, +residual stream 1.43e-3 (the GPU
 measures 1.41e-3): fp16 WEIGHT rounding alone is ~0.9e-3 rel-L2, so an fp16 tensor-core UNet
 cannot reach 1e-3 on embeddings; scores stay < 1e-3 and the ranking is unchanged."""
-import sys, torch, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, torch, numpy as np
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import torch.nn.functional as F
 from oracle import unet_oracle as orc, weights
 torch.set_num_threads(8)
 sd = weights.make_unet_state_dict(0)
-g=np.load('/root/repo/tests/golden/cfg1_b1_n6.npz')
+g=np.load(os.path.join(ROOT, 'tests', 'golden', 'cfg1_b1_n6.npz'))
 rf=torch.from_numpy(g['ref_feat']); poses=torch.from_numpy(g['all_relativeR'])[0,:2]
 x=rf.expand(2,-1,-1,-1)
 ref=orc.unet_forward(sd,x,poses)

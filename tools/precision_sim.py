@@ -14,13 +14,15 @@ round their raw output):
 
 usage: python tools/precision_sim.py [n_hyp] [bf16]
 """
+import os
 import sys
 
 import numpy as np
 import torch
 import torch.nn.functional as F
 
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 from oracle import unet_oracle as orc, weights  # noqa: E402
 
 torch.set_num_threads(8)
@@ -114,7 +116,7 @@ def main():
     dtype = torch.bfloat16 if "bf16" in sys.argv else torch.float16
     R = make_round(dtype)
     sd = weights.make_unet_state_dict(0)
-    g = np.load("/root/repo/tests/golden/level2_642_b1.npz")
+    g = np.load(os.path.join(ROOT, "tests", "golden", "level2_642_b1.npz"))
     rf = torch.from_numpy(g["ref_feat"])
     poses = torch.from_numpy(g["all_relativeR"])[0]
     pick = torch.linspace(0, 641, n).long()
