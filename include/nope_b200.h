@@ -284,6 +284,29 @@ int nope_ldm_run_block(nope_ldm_t* m, const char* name, const float* x0, int C0,
 int nope_op_mh_attention(int impl, const float* qkv, float* out, int n_img, int n_tok, int C,
                          void* stream);
 
+/* ---- VSD evaluation (src/poses/vsd.py, vsd_utils.py; the tless_<cat> branch of model.py:391-541) ----
+ * Mesh table: vertices [sum V, 3] fp32 and faces [sum F, 3] int32 (indices local to their mesh) of M
+ * meshes packed back to back; mesh_voff / mesh_foff (HOST, int64 [M + 1], starting at 0) delimit them.
+ * Render p draws mesh mesh_ids[p] (HOST, int32 [P]) under poses [P, 3, 4] fp32 (R | t, object -> OpenCV
+ * camera: x right, y down, z forward) with intrinsics [P, 4] float64 (fx, fy, cx, cy).  Pixel (x, y)
+ * samples the image point (x + 0.5, y + 0.5); depth [P, H, W] fp32 is the camera z of the nearest
+ * surface with znear <= z <= zfar, 0 where nothing is hit.  No back-face culling.  Renders are
+ * bit-reproducible and independent of how they are grouped into calls.
+ * nope_vsd_workspace_bytes returns the device workspace nope_vsd_render needs (negative on error). */
+int64_t nope_vsd_workspace_bytes(const int64_t* mesh_voff, const int64_t* mesh_foff, int M, const int* mesh_ids,
+                                 int P);
+int nope_vsd_render(const float* verts, const int* faces, const int64_t* mesh_voff, const int64_t* mesh_foff, int M,
+                    const int* mesh_ids, const float* poses, const double* intrinsics, int P, int H, int W,
+                    float znear, float zfar, void* workspace, int64_t workspace_bytes, float* depth, void* stream);
+/* VSD errors of F frames x k hypotheses (vsd_obj, vsd.py:58-136, bop19 visibility, step cost):
+ *   depth_raw [F, H, W] uint16 sensor depth, divided by depth_scale in float64 (T-LESS: 10.0 -> mm);
+ *   intrinsics [F, 4] float64 (fx, fy, cx, cy); depth_gt [F, H, W] and depth_est [F, k, H, W] fp32 renders.
+ * out_counts [F, k, 3] int64 = (|union|, |intersection|, pixels of the intersection with cost 1);
+ * out_err [F, k] float64 = (costs + |union| - |inter|) / |union|, 1.0 when the union is empty. */
+int nope_vsd_error(const uint16_t* depth_raw, double depth_scale, const double* intrinsics, const float* depth_gt,
+                   const float* depth_est, int F, int k, int H, int W, float delta, double tau, int64_t* out_counts,
+                   double* out_err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

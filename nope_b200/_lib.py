@@ -77,6 +77,12 @@ SIGNATURES = {
     "nope_op_mh_attention": (C.c_int, [C.c_int, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "nope_unet_debug_tap": (C.c_int, [C.c_void_p, c_f32p, c_f32p, C.c_int, C.c_char_p, c_f32p,
                                       C.c_int64, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]),
+    "nope_vsd_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int]),
+    "nope_vsd_render": (C.c_int, [c_f32p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, c_f32p, C.c_void_p,
+                                  C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_int64, c_f32p,
+                                  C.c_void_p]),
+    "nope_vsd_error": (C.c_int, [C.c_void_p, C.c_double, C.c_void_p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int,
+                                 C.c_int, C.c_float, C.c_double, c_i64p, C.c_void_p, C.c_void_p]),
 }
 
 EXPECTED_ABI = 2     # include/nope_b200.h "ABI version"; a stale build with other signatures must not bind

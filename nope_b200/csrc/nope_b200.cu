@@ -23,6 +23,7 @@
 #include "linattn_tc.cuh"
 #include "encoder.cuh"
 #include "ldm.cuh"
+#include "vsd.cuh"
 
 using namespace nope;
 
@@ -2029,6 +2030,124 @@ int nope_op_mh_attention(int impl, const float* qkv, float* out, int n_img, int 
   nhwc_f16_to_nchw_f32_kernel<<<ew_grid((long long)tok * C), 256, 0, st>>>(o16, out, (int)tok, C, 1);
   NOPE_CUDA(cudaGetLastError());
   NOPE_CUDA(cudaStreamSynchronize(st));
+  return 0;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------
+// VSD evaluation: depth renders + fused VSD error (vsd.cuh)
+// ---------------------------------------------------------------------------------
+namespace {
+struct VsdLayout {
+  size_t info, cam, big, counter, total;
+};
+int vsd_plan(const int64_t* mesh_voff, const int64_t* mesh_foff, int M, const int* mesh_ids, int P,
+             std::vector<VsdRenderInfo>* infos, VsdLayout* L) {
+  NOPE_CHECK(mesh_voff && mesh_foff && mesh_ids, "null argument");
+  NOPE_CHECK(M >= 1 && P >= 1 && P <= 65535, "need M >= 1 meshes and 1 <= P <= 65535 renders");
+  NOPE_CHECK(mesh_voff[0] == 0 && mesh_foff[0] == 0, "mesh offsets must start at 0");
+  for (int m = 0; m < M; ++m) {
+    NOPE_CHECK(mesh_voff[m + 1] > mesh_voff[m] && mesh_foff[m + 1] > mesh_foff[m],
+               "mesh offsets must increase strictly (every mesh needs vertices and faces)");
+    NOPE_CHECK(mesh_voff[m + 1] - mesh_voff[m] <= INT32_MAX && mesh_foff[m + 1] - mesh_foff[m] <= INT32_MAX,
+               "a mesh has more than 2^31 - 1 vertices or faces");
+  }
+  long long nv = 0, nf = 0;
+  if (infos) infos->resize(P);
+  for (int p = 0; p < P; ++p) {
+    const int m = mesh_ids[p];
+    NOPE_CHECK(m >= 0 && m < M, "mesh id " + std::to_string(m) + " of render " + std::to_string(p) +
+                                    " is outside [0, " + std::to_string(M) + ")");
+    VsdRenderInfo ri;
+    ri.nv = (int)(mesh_voff[m + 1] - mesh_voff[m]);
+    ri.nf = (int)(mesh_foff[m + 1] - mesh_foff[m]);
+    ri.vbase = mesh_voff[m];
+    ri.fbase = mesh_foff[m];
+    ri.wbase = nv;
+    if (infos) (*infos)[p] = ri;
+    nv += ri.nv;
+    nf += ri.nf;
+  }
+  auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
+  L->info = 0;
+  L->cam = up(sizeof(VsdRenderInfo) * (size_t)P);
+  L->big = L->cam + up(sizeof(double) * 3 * (size_t)nv);
+  L->counter = L->big + up(sizeof(int2) * (size_t)nf);
+  L->total = L->counter + 256;
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int64_t nope_vsd_workspace_bytes(const int64_t* mesh_voff, const int64_t* mesh_foff, int M, const int* mesh_ids,
+                                 int P) {
+  VsdLayout L;
+  if (vsd_plan(mesh_voff, mesh_foff, M, mesh_ids, P, nullptr, &L)) return -1;
+  return (int64_t)L.total;
+}
+
+int nope_vsd_render(const float* verts, const int* faces, const int64_t* mesh_voff, const int64_t* mesh_foff, int M,
+                    const int* mesh_ids, const float* poses, const double* intrinsics, int P, int H, int W,
+                    float znear, float zfar, void* workspace, int64_t workspace_bytes, float* depth, void* stream) {
+  NOPE_CHECK(H >= 1 && W >= 1 && (int64_t)H * W <= INT32_MAX, "image size must satisfy 1 <= H*W <= 2^31 - 1");
+  NOPE_CHECK(verts && faces && poses && intrinsics && depth, "null argument");
+  NOPE_CHECK(znear > 0.f && zfar > znear, "need 0 < znear < zfar");
+  std::vector<VsdRenderInfo> infos;
+  VsdLayout L;
+  if (vsd_plan(mesh_voff, mesh_foff, M, mesh_ids, P, &infos, &L)) return -1;
+  NOPE_CHECK(workspace && workspace_bytes >= (int64_t)L.total,
+             "workspace smaller than nope_vsd_workspace_bytes (" + std::to_string(L.total) + " bytes)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  char* ws = static_cast<char*>(workspace);
+  auto* info = reinterpret_cast<VsdRenderInfo*>(ws + L.info);
+  auto* cam = reinterpret_cast<double*>(ws + L.cam);
+  auto* big = reinterpret_cast<int2*>(ws + L.big);
+  auto* n_big = reinterpret_cast<unsigned int*>(ws + L.counter);
+  NOPE_CUDA(cudaMemcpyAsync(info, infos.data(), sizeof(VsdRenderInfo) * P, cudaMemcpyHostToDevice, st));
+  NOPE_CUDA(cudaMemsetAsync(n_big, 0, sizeof(unsigned int), st));
+  int max_nv = 0, max_nf = 0;
+  for (const auto& ri : infos) {
+    max_nv = std::max(max_nv, ri.nv);
+    max_nf = std::max(max_nf, ri.nf);
+  }
+  const size_t n_px = (size_t)P * H * W;
+  auto* zbuf = reinterpret_cast<unsigned int*>(depth);
+  const int ew = (int)std::min<size_t>((n_px + 255) / 256, 4096);
+  vsd_fill_kernel<<<ew, 256, 0, st>>>(zbuf, n_px, 0x7f800000u);
+  NOPE_CUDA(cudaGetLastError());
+  vsd_vertex_kernel<<<dim3(std::min((max_nv + 255) / 256, 1024), P), 256, 0, st>>>(verts, poses, info, cam);
+  NOPE_CUDA(cudaGetLastError());
+  vsd_face_kernel<<<dim3((max_nf + 127) / 128, P), 128, 0, st>>>(faces, cam, info, intrinsics, H, W, znear, zfar,
+                                                                 zbuf, big, n_big);
+  NOPE_CUDA(cudaGetLastError());
+  vsd_big_face_kernel<<<kVsdBigTriCtas, 256, 0, st>>>(faces, cam, info, intrinsics, H, W, znear, zfar, zbuf, big,
+                                                       n_big);
+  NOPE_CUDA(cudaGetLastError());
+  vsd_finish_kernel<<<ew, 256, 0, st>>>(zbuf, n_px);
+  NOPE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int nope_vsd_error(const uint16_t* depth_raw, double depth_scale, const double* intrinsics, const float* depth_gt,
+                   const float* depth_est, int F, int k, int H, int W, float delta, double tau, int64_t* out_counts,
+                   double* out_err, void* stream) {
+  NOPE_CHECK(depth_raw && intrinsics && depth_gt && depth_est && out_counts && out_err, "null argument");
+  NOPE_CHECK(F >= 1 && F <= 65535 && k >= 1 && k <= 65535 && (int64_t)F * k <= INT32_MAX,
+             "need 1 <= F, k <= 65535 and F*k <= 2^31 - 1");
+  NOPE_CHECK(H >= 1 && W >= 1 && (int64_t)H * W <= INT32_MAX, "image size must satisfy 1 <= H*W <= 2^31 - 1");
+  NOPE_CHECK(depth_scale > 0.0, "depth_scale must be positive");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  NOPE_CUDA(cudaMemsetAsync(out_counts, 0, sizeof(int64_t) * 3 * (size_t)F * k, st));
+  const int slices = (int)(((int64_t)H * W + kVsdErrPixelsPerCta - 1) / kVsdErrPixelsPerCta);
+  vsd_error_kernel<<<dim3(slices, k, F), 256, 0, st>>>(depth_raw, depth_scale, intrinsics, depth_gt, depth_est, k,
+                                                       H, W, delta, tau,
+                                                       reinterpret_cast<unsigned long long*>(out_counts));
+  NOPE_CUDA(cudaGetLastError());
+  vsd_error_finish_kernel<<<(F * k + 255) / 256, 256, 0, st>>>(
+      reinterpret_cast<const unsigned long long*>(out_counts), F * k, out_err);
+  NOPE_CUDA(cudaGetLastError());
   return 0;
 }
 

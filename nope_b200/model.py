@@ -1,8 +1,8 @@
 """Host-side mirror of the reference task module `PoseConditional`
 (src/model/model.py:32-565), inference surface only: forward (loss), sample,
 generate_templates, retrieval, plus predict_pose (= eval_geodesic lines 313-357 without
-logging, SURVEY.md F2).  Training, VSD evaluation, wandb/video logging are out of scope
-(SURVEY.md section 8).
+logging, SURVEY.md F2), and the T-LESS evaluation eval_vsd (model.py:378-541) on the GPU renderer and
+VSD kernel of nope_b200.vsd.  Training, wandb/video logging are out of scope (SURVEY.md section 8).
 
 Differences that are deliberate and documented:
   * generate_templates batches the whole pose grid through one engine sweep instead of a
@@ -10,8 +10,11 @@ Differences that are deliberate and documented:
   * retrieval raises ValueError for an unknown metric instead of returning None
     (model.py:256 falls through); "cosine" is an extension (SURVEY.md F3).
   * ranking is deterministic: descending score, ties -> lowest index.
+  * eval_vsd follows vsd_obj's per-frame contract (vsd.py:58-136); the reference's eval_vsd cannot run as
+    written (see nope_b200/vsd.py).  Errors come back in frame order, the GT pose is rendered once per frame.
 """
 import ctypes as C
+import os
 import types
 
 import torch
@@ -171,14 +174,73 @@ class PoseConditional:
                      nearest_idx=nearest_idx.cpu().numpy())
         return error, nearest_idx, similarity
 
+    # ------------------------------------------------------------------ model.py:378-389
+    def load_mesh(self, cad_dir, obj_ids=range(1, 31)):
+        """The T-LESS CAD models obj_000001.ply ... obj_000030.ply (mm), packed on the model's device."""
+        from .vsd import MeshTable
+        self.tless_obj_ids = list(obj_ids)
+        self.tless_cad = MeshTable([os.path.join(cad_dir, f"obj_{i:06d}.ply") for i in self.tless_obj_ids],
+                                   device=self.device)
+        return self
+
+    # ------------------------------------------------------------------ model.py:391-541
+    @torch.no_grad()
+    def eval_vsd(self, batch, data_name, save_path=None):
+        """`eval_vsd` of the reference without the wandb / image logging and the process pool: validation
+        loss, top-5 retrieval (through ShardedSweep when set; every rank then computes the same VSD),
+        predicted poses = retrieved rotations with the GT translation, 1 + k depth renders per frame, VSD
+        errors [B,k] (float64), the scores of model.py:530-537.  Saves vsd_error[:, 0] to `save_path`."""
+        import numpy as np
+        from .vsd import render_depth, vsd_error, vsd_scores
+        if getattr(self, "tless_cad", None) is None:
+            raise RuntimeError("eval_vsd needs the CAD models: call load_mesh(cad_dir) first")
+        query, reference = batch["query"], batch["reference"]
+        loss = self.forward(query=query, relativeR=batch["gt_relativeR"], reference=reference)
+        self.log(f"loss/val_{data_name}", loss)
+        _, nearest_idx, _ = self.predict_pose(query, reference, batch["all_relativeR"], None, k=5)
+        dev = nearest_idx.device
+        B, k = nearest_idx.shape
+        tp = batch["template_poses"].to(dev)
+        retrieved_R = tp[torch.arange(B, device=dev)[:, None].expand(B, k), nearest_idx]   # model.py:469-475
+        t = batch["query_translation"].to(dev, torch.float32).reshape(B, 3, 1)
+        gt = torch.cat([batch["query_pose"].to(dev, torch.float32), t], dim=2)           # [B,3,4]
+        pred = torch.cat([retrieved_R.to(torch.float32), t[:, None].expand(B, k, 3, 1)], dim=3)
+        obj_ids = [int(i) for i in torch.as_tensor(batch["obj_id"]).reshape(-1).tolist()]
+        try:
+            mesh_idx = [self.tless_obj_ids.index(i) for i in obj_ids]
+        except ValueError:
+            raise ValueError(f"obj_id {obj_ids} not among the loaded meshes {self.tless_obj_ids}") from None
+        if "depth_raw" in batch:
+            depth_raw = batch["depth_raw"].to(dev)
+        else:
+            from .tless import read_depth
+            depth_raw = read_depth(batch["depth_path"]).to(dev)
+        H, W = depth_raw.shape[-2:]
+        K = batch["intrinsic"].to(dev)
+        poses = torch.cat([gt[:, None], pred], dim=1).reshape(B * (1 + k), 3, 4)
+        ids = [m for m in mesh_idx for _ in range(1 + k)]
+        depth = render_depth(self.tless_cad, ids, poses, K.double().repeat_interleave(1 + k, 0), H, W)
+        depth = depth.view(B, 1 + k, H, W)
+        err = vsd_error(depth_raw, K.double(), depth[:, 0], depth[:, 1:])
+        scores = vsd_scores(err)
+        self.log_score(scores, split_name=f"val_{data_name}")
+        err = err.cpu().numpy()
+        if save_path is not None:
+            os.makedirs(os.path.dirname(os.path.abspath(save_path)), exist_ok=True)
+            np.save(save_path, err[:, 0])
+        self.last_vsd_error = err
+        return scores
+
     def test_step(self, batch, idx_batch):
         """model.py:550-565: one entry per dataloader, keyed "<dataset>_<category>"."""
         out = {}
         for dataloader_name in batch.keys():
             data_name, category = dataloader_name.split("_")
             if data_name in ["tless"]:
-                raise ValueError("the T-LESS / VSD evaluation (eval_vsd, pyrender) is outside this package's "
-                                 "scope (SURVEY.md section 2): only shapeNet_<category> dataloaders are handled")
+                save_path = None if self.save_dir is None else os.path.join(
+                    self.save_dir, "predictions", f"vsd_{category}_batch{idx_batch}_rank_{self.global_rank}.npy")
+                out[dataloader_name] = self.eval_vsd(batch[dataloader_name], category, save_path=save_path)
+                continue
             out[dataloader_name] = self.eval_geodesic(batch[dataloader_name], category, visualize=True,
                                                       save_prediction=True)
         self.global_step += 1
